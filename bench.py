@@ -6,6 +6,7 @@
   torchrun --nproc-per-node N bench.py --gpus N ...        one process per GPU, prompt-sharded replicas
 
   ... --workload image|refiner|inpaint                     whole images through sdxl_sample_latent (BASELINE configs 3, 4, 5)
+  ... --dump-outputs DIR                                   also write the last timed step's result (rank 0) as DIR/latent.npy
 
 A "step" = one iteration of the reference's sampler loop body (src/model/stablediffusion/mod.rs:406-429):
 alpha lookups, forward_diffuser (conditional + unconditional UNet evaluation, CFG combine) and the DDIM
@@ -30,6 +31,7 @@ for p in (ROOT, PKG):
     if p not in sys.path:
         sys.path.insert(0, p)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 METRIC = "unet_sampler_steps_per_sec_1024x1024_bs1"
@@ -102,6 +104,14 @@ class ClockSampler:
             except Exception:
                 pass
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": mx or None, "reasons": sorted(reasons), "samples": len(sm)}
+
+
+def dump_outputs(directory, **arrays):
+    """`--dump-outputs`: what the timed path returned in its last step, one float32 .npy per array, so that two builds run with
+    the same arguments (hence the same seeded inputs) can be compared output for output."""
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), t.detach().float().cpu().numpy())
 
 
 def make_conditioning(rank: int, device):
@@ -287,7 +297,7 @@ def run_ours(args, rank: int, local_rank: int, world: int):
     # the value is built on the MEDIAN step (the box's host cores are shared: a single preemption of tens of ms inside a 0.2 s
     # region would otherwise halve the number; the mean is reported beside it). Runs before the clock sampler's nvidia-smi starts.
     host_lat = torch.randn(1, 4, HW // 8, HW // 8).pin_memory()
-    e2e_steps = max(3, args.steps)
+    e2e_steps = args.steps
     for _ in range(2):
         diffuser.sampler_step_host(999, 999 - step_size, host_lat)
     barrier()
@@ -322,6 +332,8 @@ def run_ours(args, rank: int, local_rank: int, world: int):
     torch.cuda.nvtx.range_pop()
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, latent=diffuser.sampler_get_latent(torch.empty(1, 4, HW // 8, HW // 8)))
     ms_total = e0.elapsed_time(e1)
     launches = ctx.launch_count - launches0
     ms_step = sharding.max_over_ranks(ms_total, dev) / args.steps   # timing rule: max over ranks of the device time
@@ -477,11 +489,13 @@ def run_images(args, rank, local_rank, world, ctx, base, refiner, dist, comm, lo
     sampler.start()
     e0.record(ctx.stream)
     for _ in range(args.steps):
-        one_image()
+        out = one_image()
     e1.record(ctx.stream)
     ctx.synchronize()
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, latent=out)
     ms_img = sharding.max_over_ranks(e0.elapsed_time(e1), dev) / args.steps
     value = world * 1e3 / ms_img
     launches = ctx.launch_count - launches0
@@ -536,7 +550,13 @@ def main():
     ap.add_argument("--workload", default="step", choices=["step", "image", "refiner", "inpaint"],
                     help="step (default): BASELINE metric, sampler steps/s at 1024^2 bs=1; image / refiner / inpaint: whole images (configs 3 / 4 / 5)")
     ap.add_argument("--dump-ops", default=None, help="write a per-launch CSV of one step (CUDA-event times)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write the final latent of the last one (rank 0, float32) as DIR/latent.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.warmup < 3 and args.workload == "step":
         args.warmup = 3
     rank = int(os.environ.get("RANK", "0"))
@@ -549,7 +569,8 @@ def main():
         # launched without torchrun: re-exec under torch.distributed.run
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}", "--master-addr", "127.0.0.1",
                "--master-port", os.environ.get("MASTER_PORT", "29541"), os.path.abspath(__file__), "--gpus", str(args.gpus), "--steps", str(args.steps),
-               "--warmup", str(args.warmup), "--workload", args.workload] + (["--no-cpu-baseline"] if args.no_cpu_baseline else [])
+               "--warmup", str(args.warmup), "--workload", args.workload] + (["--no-cpu-baseline"] if args.no_cpu_baseline else []) \
+            + (["--dump-outputs", os.path.abspath(args.dump_outputs)] if args.dump_outputs else [])
         sys.exit(subprocess.call(cmd))
     run_ours(args, rank, local_rank, world)
 

@@ -2,9 +2,10 @@
 
 Pinning chain: the reference's known-answer vector (src/token/clip.rs:232-249) pins the Python oracle
 (oracle/tokenizer_oracle.py, a line-by-line restatement); the oracle generated tests/golden/tokenizer_vectors.json; the C++
-tokenizer must reproduce those vectors and agree with the oracle on a seeded fuzz corpus. Tests that need the reference's
-vocabulary files (3 MB of third-party data that is not copied into this repo) look in $SDXL_TOKENIZER_DIR or
-/root/reference/tokenizer and skip when absent; the mini-vocabulary tests run everywhere. CPU only, no GPU call.
+tokenizer must reproduce those vectors and agree with the oracle on a seeded fuzz corpus. The real CLIP / OpenCLIP vocabularies
+(3 MB of third-party data) are not stored whole: tests/golden/tokenizer_ref_subset.json keeps every entry this file's corpus
+reaches at its original position (tests/golden/make_tokenizer_golden.py says why that tokenizes the corpus exactly as the full
+files do), and the `real` fixture writes it back out as vocabulary files. CPU only, no GPU call.
 """
 import json
 import os
@@ -18,9 +19,6 @@ from sdxl_b200 import SdxlError
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 MINI = os.path.join(GOLD, "mini_bpe")
-REF_TOK = os.environ.get("SDXL_TOKENIZER_DIR", "/root/reference/tokenizer")
-HAVE_REF = os.path.exists(os.path.join(REF_TOK, "clip", "bpe_simple_vocab_16e6.txt"))
-need_ref = pytest.mark.skipif(not HAVE_REF, reason="reference vocabulary files not present")
 VEC = json.load(open(os.path.join(GOLD, "tokenizer_vectors.json"), encoding="utf-8"))
 
 KAT_TEXT = "Hello world! <|startoftext|>asdf<|startoftext|>"
@@ -34,14 +32,24 @@ def mini():
             TO.OpenClipTokenizer(os.path.join(MINI, "mini_merges.txt"), os.path.join(MINI, "mini_vocab.txt")))
 
 
+def _write_subset(path, table, placeholder):
+    """One line per position: the kept entry, or a placeholder on U+E000 that no byte-level piece can equal."""
+    keep = table["keep"]
+    with open(path, "w", encoding="utf-8", newline="\n") as f:
+        f.writelines((keep[str(i)] if str(i) in keep else placeholder(i)) + "\n" for i in range(table["n"]))
+    return path
+
+
 @pytest.fixture(scope="module")
-def real():
-    c = os.path.join(REF_TOK, "clip", "bpe_simple_vocab_16e6.txt")
-    m, v = os.path.join(REF_TOK, "open_clip", "merges.txt"), os.path.join(REF_TOK, "open_clip", "vocab.txt")
+def real(tmp_path_factory):
+    sub = json.load(open(os.path.join(GOLD, "tokenizer_ref_subset.json"), encoding="utf-8"))
+    d = tmp_path_factory.mktemp("ref_vocab")
+    c = _write_subset(str(d / "bpe_simple_vocab_16e6.txt"), sub["clip_merges"], lambda i: f"\ue000{i} \ue001")
+    m = _write_subset(str(d / "merges.txt"), sub["open_clip_merges"], lambda i: f"\ue000{i} \ue001")
+    v = _write_subset(str(d / "vocab.txt"), sub["open_clip_vocab"], lambda i: f"\ue000{i}")
     return {"clip": (ClipTokenizer(c), TO.ClipTokenizer(c)), "open_clip": (OpenClipTokenizer(m, v), TO.OpenClipTokenizer(m, v))}
 
 
-@need_ref
 def test_reference_known_answer_pins_the_oracle(real):
     """src/token/clip.rs:232-249, verbatim."""
     _, oracle = real["clip"]
@@ -50,7 +58,6 @@ def test_reference_known_answer_pins_the_oracle(real):
     assert oracle.decode(enc) == KAT_DECODE
 
 
-@need_ref
 def test_reference_known_answer_cxx(real):
     tok, _ = real["clip"]
     enc = tok.encode(KAT_TEXT, False, False)
@@ -61,7 +68,6 @@ def test_reference_known_answer_cxx(real):
     assert otok.padding_token() == 0   # open_clip.rs:218-220
 
 
-@need_ref
 @pytest.mark.parametrize("which", ["clip", "open_clip"])
 def test_real_vocab_vectors(real, which):
     tok, oracle = real[which]
@@ -125,7 +131,6 @@ def test_fuzz_cxx_equals_oracle_mini(mini):
     assert n == 400
 
 
-@need_ref
 def test_fuzz_cxx_equals_oracle_real(real):
     for which in ("clip", "open_clip"):
         tok, oracle = real[which]
@@ -175,19 +180,12 @@ def test_invalid_utf8_is_replaced_like_from_utf8_lossy(mini):
         assert list(buf[:n.value]) == oracle.encode(raw.decode("utf-8", errors="replace"), False, False), raw
 
 
-@need_ref
 def test_open_clip_ids_match_huggingface_tokenizers(real):
-    """Independent check: the HuggingFace `tokenizers` runtime on the reference's own tokenizer.json (the file its
-    vocab.txt / merges.txt were exported from, tokenizer/convert.py) gives the same ids as the oracle and the C++ tokenizer
-    (NFC-stable prompts: tokenizer.json normalises with NFC, the reference's Rust code does not)."""
-    tk = pytest.importorskip("tokenizers")
-    path = os.path.join(REF_TOK, "tokenizer.json")
-    if not os.path.exists(path):
-        pytest.skip("tokenizer.json not present")
-    hf = tk.Tokenizer.from_file(path)
+    """Independent check: the ids the HuggingFace `tokenizers` runtime gives on the reference's own tokenizer.json (the file
+    its vocab.txt / merges.txt were exported from, tokenizer/convert.py; stored in the vectors file) equal those of the oracle
+    and the C++ tokenizer (NFC-stable prompts: tokenizer.json normalises with NFC, the reference's Rust code does not)."""
     tok, oracle = real["open_clip"]
-    for p in ["a photo of a cat", "An astronaut riding a horse on Mars, 4k, highly-detailed!!",
-              "it's the artist's 1st painting; they've said we'll see", "Ünïcödé façade naïve café", "x²+y³ = 42 %"]:
-        want = hf.encode(p).ids            # adds <|startoftext|> / <|endoftext|>
+    hf = VEC["huggingface_open_clip"]
+    for p, want in zip(hf["prompts"], hf["encode"]):   # want includes <|startoftext|> / <|endoftext|>
         assert oracle.encode(p, True, True) == want, p
         assert tok.encode(p, True, True) == want, p

@@ -1,7 +1,6 @@
-"""The tokenizer parity tests again under the `gpu` marker, so the GPU-box test record shows them (they need no GPU; the default
-`-m gpu` selection would otherwise deselect the whole tokenizer suite). Vocabulary-independent cases run everywhere; the cases that
-need the reference's vocabulary files (the known-answer vector of src/token/clip.rs:232-249 among them) run where
-SDXL_TOKENIZER_DIR / /root/reference/tokenizer exists and skip on the GPU box, which has no copy of the reference."""
+"""The tokenizer parity tests again under the `gpu` marker, so a `-m gpu` run includes them (they need no GPU; that selection
+would otherwise deselect the whole tokenizer suite). The real-vocabulary cases (the known-answer vector of
+src/token/clip.rs:232-249 among them) run on the stored vocabulary subset, like everything else in test_tokenizer.py."""
 import pytest
 
 import test_tokenizer as T
