@@ -173,6 +173,48 @@ SDXL_API int sdxl_dbg_igemm_timeline(sdxl_ctx* ctx, int M, int K, int N, int geg
                                      uint64_t* stamps_host);
 /* Diagnostics: clock stamps of CTA 0 of one attention launch on synthetic data; stamps_host[3][256][4] (csrc/engine.cu). */
 SDXL_API int sdxl_dbg_attention_timeline(sdxl_ctx* ctx, int B, int T, int S, int n_head, long long* stamps_host);
+/* Diagnostics: the launch builders of the UNet / VAE / CLIP plans on caller data, for direct kernel tests. Each call builds a
+ * scratch plan (weights re-laid out from a pack exactly as the model loaders do), runs it once on the ctx stream and waits.
+ * Device pointers except `pack` (host, the sdxl_unet_load format). cfg_out (nullable, host): per implicit-GEMM launch
+ * SDXL_DBG_CFG_FIELDS ints {pair, CM, CN, a_split_dim, BN, nstages, epi_tma, epi_box_bytes}; unused rows up to cfg_cap = -1.
+ * kind (pack tensor names; shapes as the model packs):
+ *   SDXL_DBG_CONV3      ResBlock 3x3 conv, "conv" [Cout,Cin,3,3] (+ "skip" [Cout,C2,1,1] fused as K columns on x2 when C2 > 0):
+ *                       x f16 [B,H,W,Cin], x2 f16 [B,H,W,C2]; bias = bias_rows + bias_off with row stride bias_ld per image
+ *                       (f32, the per-image time-embedding bias) or the conv bias when bias_rows is NULL; residual f32
+ *                       [B*H*W, Cout] or NULL; out f32 [B*H*W, Cout] (ldo unused)
+ *   SDXL_DBG_UPCONV     nearest-2x + 3x3 conv as four phase convs: x f32 [B,H,W,Cin] -> out f32 [B,2H,2W,Cout]
+ *   SDXL_DBG_HEAD_HILO  output head GN(32) -> SiLU -> 3x3 conv on the hi/lo-split activation, "norm" + "conv":
+ *                       x f32 [B,H,W,Cin] -> out f32 [B*H*W, ldo]
+ *   SDXL_DBG_PADDED_S2  PaddedConv2d 3x3 stride 2, zero pad bottom / right: x f32 [B,H,W,Cin] -> out f32 [B,H/2,W/2,Cout]
+ *   SDXL_DBG_LINEAR / _LINEAR_F16 / _GEGLU   PlanBuilder::linear, "lin" [Cin,Cout] + bias: x f16 [W, Cin] (B = H = 1),
+ *                       out [W, ldo] f32 / f16 / f16 GEGLU (Cout = fused 2*n_out); residual f32 [W, ldo] or NULL */
+#define SDXL_DBG_CFG_FIELDS 8
+#define SDXL_DBG_CONV3 0
+#define SDXL_DBG_UPCONV 1
+#define SDXL_DBG_HEAD_HILO 2
+#define SDXL_DBG_PADDED_S2 3
+#define SDXL_DBG_LINEAR 4
+#define SDXL_DBG_LINEAR_F16 5
+#define SDXL_DBG_GEGLU 6
+SDXL_API int sdxl_dbg_plan_gemm(sdxl_ctx* ctx, int kind, const void* pack_host, size_t pack_bytes, int B, int H, int W, int Cin,
+                                int Cout, int C2, const void* x, const void* x2, const float* bias_rows, int bias_ld, int bias_off,
+                                const float* residual, void* out, int ldo, int32_t* cfg_out_host, int cfg_cap);
+/* GroupNorm(32) as the ResBlocks and the head record it: "norm" [C1+C2]; x1 f32 [B,HW,C1], x2 (nullable) [B,HW,C2]; y f16
+ * [B,HW,C1+C2]; raw (nullable) f16(cat(x1,x2)); y_lo (nullable) f16(t - y), the rounding residue of y. */
+SDXL_API int sdxl_dbg_plan_group_norm(sdxl_ctx* ctx, const void* pack_host, size_t pack_bytes, const float* x1, int C1,
+                                      const float* x2, int C2, int B, int HW, int silu, sdxl_half* y, sdxl_half* raw,
+                                      sdxl_half* y_lo);
+/* Attention on column windows as the plans record it: q at columns q_col0.. of [B*T, q_pitch]; k / v at k_col0 / v_col0 of one
+ * [B*S, kv_pitch] matrix; out [B*T, ldo]; head dim 64. small != 0: the short-sequence kernel (additive f16 mask [T,S] or NULL,
+ * causal), else the tensor-core kernel (mask / causal ignored). */
+SDXL_API int sdxl_dbg_plan_attention(sdxl_ctx* ctx, int small, const sdxl_half* q, int q_pitch, int q_col0, const sdxl_half* kv,
+                                     int kv_pitch, int k_col0, int v_col0, int B, int T, int S, int n_head, const sdxl_half* mask,
+                                     int causal, sdxl_half* out, int ldo);
+/* The VAE's single-head attention of one image: q, k, v f16 [T,C] -> scores f32 [T,T] = q k^T, probs f16 [T,T] =
+ * softmax(scores / sqrt(C)), vT f16 [C,T], out f16 [T,C] = probs v. T, C multiples of 64. */
+SDXL_API int sdxl_dbg_plan_vae_attention(sdxl_ctx* ctx, const sdxl_half* q, const sdxl_half* k, const sdxl_half* v, int T, int C,
+                                         float* scores, sdxl_half* probs, sdxl_half* vT, sdxl_half* out, int32_t* cfg_out_host,
+                                         int cfg_cap);
 /* seeded N(0,1) exactly as the sampler generates it (device out). */
 SDXL_API int sdxl_randn(sdxl_ctx* ctx, float* out, size_t n, uint64_t seed, uint64_t subsequence);
 

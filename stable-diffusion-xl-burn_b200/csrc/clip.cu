@@ -175,13 +175,7 @@ static int build_clip_plan(sdxl_clip* m, Plan* P, Arena* A, int n_run, int captu
     // x = x + attn(attn_ln(x), causal mask)    (clip/mod.rs:177-179)
     B.ln(x, b.attn_ln, M, a16);
     B.linear(a16, M, b.qkv, IGEMM_LINEAR, qkv16, 0, 3 * C, nullptr, 0);
-    {
-      Op op{};
-      op.kind = OP_ATTN_SMALL;
-      op.as = {qkv16, 3 * C, 0, qkv16, qkv16, 3 * C, C, 2 * C, Bn, T, T, g.n_head, nullptr, 1, ao16, C};
-      P->ops.push_back(op);
-      B.add_flops(4.0 * Bn * T * (double)T * C);
-    }
+    B.attn_small(qkv16, 3 * C, 0, qkv16, 3 * C, C, 2 * C, T, T, g.n_head, nullptr, 1, ao16, C);
     B.linear(ao16, M, b.out, IGEMM_LINEAR, xn, 1, C, x, C);
     // x = x + mlp(mlp_ln(x))
     B.ln(xn, b.mlp_ln, M, a16);

@@ -297,15 +297,8 @@ static int build_model(sdxl_unet* u, const PackView& pv, Arena& A) {
   if (L.err) return L.err;
   // The head conv is the one GEMM whose operand-rounding error reaches eps undamped (every other layer's is averaged by what
   // follows), so its activation operand is split hi + lo (two f16 tensors, ~22 bits): same weights twice along K.
-  {
-    const Conv& cv = u->conv_out;
-    u->conv_out_w2 = A.get<__half>((size_t)cv.O * 2 * cv.Ktot);
-    if (!u->conv_out_w2) return fail(c, 4005, "weight arena exhausted");
-    if (!A.measure)
-      for (int h2 = 0; h2 < 2; ++h2)
-        CU(c, cudaMemcpy2DAsync(u->conv_out_w2 + (size_t)h2 * cv.Ktot, (size_t)2 * cv.Ktot * sizeof(__half), cv.w, (size_t)cv.Ktot * sizeof(__half),
-                                (size_t)cv.Ktot * sizeof(__half), (size_t)cv.O, cudaMemcpyDeviceToDevice, c->stream));
-  }
+  u->conv_out_w2 = L.dup_k(u->conv_out);
+  if (L.err) return L.err;
 
   // concatenated lin_embed matrix (one GEMV per forward for all ResBlocks); bias += conv_in bias
   {
@@ -536,25 +529,6 @@ struct UNetPlanBuilder : PlanBuilder {
     linear(s_a16, M, s.proj_out, IGEMM_LINEAR, out, 1, C, x, C);
     return out;
   }
-  void attn(const __half* qm, int q_pitch, int q_col0, const __half* kvm, int kv_pitch, int k_col0, int v_col0, int T,
-            int S, int n_head, __half* out, int ldo, float sl2e) {
-    if (err) return;
-    Op op{};
-    op.kind = OP_ATTN;
-    AttnParams& p = op.at;
-    p.T = T; p.S = S; p.n_head = n_head; p.B = Bf;
-    p.q_col0 = q_col0; p.k_col0 = k_col0; p.v_col0 = v_col0;
-    p.out = out; p.ldo = ldo; p.scale_log2e = sl2e;
-    if (!A->measure) {
-      int r = make_tmap_rows(&p.tmQ, qm, T, Bf, q_pitch, q_pitch);
-      if (!r) r = make_tmap_rows(&p.tmK, kvm, S, Bf, kv_pitch, kv_pitch);
-      if (!r) p.tmV = p.tmK;
-      if (r) { err = fail(c, r, "tensor map creation failed (attention)"); return; }
-    }
-    op.flops_exec = 4.0 * Bf * (double)((T + 127) / 128 * 128) * (double)((S + 127) / 128 * 128) * (n_head * 64);
-    P->ops.push_back(op);
-    add_flops(4.0 * Bf * T * (double)S * (n_head * 64));
-  }
 };
 
 
@@ -702,19 +676,8 @@ static int build_plan_ops(sdxl_unet* u, Plan* P, Arena* A) {
   }
   if (B.err) return B.err;
   B.begin_block("norm_out+conv_out");
-  // --- head: GN -> SiLU -> conv 3x3 (unet/mod.rs:488-490)
-  B.gn(x, Cx, nullptr, 0, H * W, u->norm_out, 1, s_gn1, nullptr);
-  if (!B.err && !P->ops.empty()) P->ops.back().gn.y_lo = s_raw;   // rounding residue of the normalised activation (hi/lo split)
-  {
-    ActView a{s_gn1, Bf, H, W, Cx}, alo{s_raw, Bf, H, W, Cx};
-    std::vector<IgemmSeg> segs;
-    for (int part = 0; part < 2; ++part)   // K = [9 taps on hi | 9 taps on lo], weights [W | W]
-      for (int kh = 0; kh < 3; ++kh)
-        for (int kw = 0; kw < 3; ++kw) segs.push_back({(int16_t)part, (int16_t)(kw - 1), (int16_t)(kh - 1), 0, u->conv_out.Ipad / 64});
-    B.igemm(a, &alo, segs, u->conv_out_w2, u->conv_out.O, 2 * u->conv_out.Ktot, H, W, Bf, IGEMM_LINEAR, 0, P->eps, 1, P->eps_ld,
-            u->conv_out.b, 0, nullptr, 0);
-    B.add_flops(2.0 * Bf * H * W * 9.0 * Cx * u->conv_out.O);
-  }
+  // --- head: GN -> SiLU -> conv 3x3 (unet/mod.rs:488-490), hi/lo split (s_raw holds the rounding residue of the activation)
+  B.head_hilo(x, Cx, H, W, u->norm_out, u->conv_out, u->conv_out_w2, s_gn1, s_raw, P->eps, P->eps_ld);
   B.end_block();
   return B.err;
 }
@@ -1388,4 +1351,142 @@ extern "C" int sdxl_dbg_igemm_timeline(sdxl_ctx* c, int M, int K, int N, int geg
   cudaEventDestroy(e0);
   cudaEventDestroy(e1);
   return 0;
+}
+
+// ================================================================================================
+// Diagnostics: the plans' own launch builders on caller data (tests/test_plan_kernels_gpu.py)
+// ================================================================================================
+// Builds a scratch plan the way the UNet / VAE / CLIP plans are built: a measure pass sizes one arena for the weights
+// (re-laid out from `pack` by the Loader helpers) and the plan's scratch, the real pass loads and records the ops, and the
+// plan's op executor runs them once (eager). `body(L, B)` loads its weights and records its ops; it runs in both passes.
+template <typename F>
+static int run_scratch_plan(sdxl_ctx* c, const void* pack, size_t pack_bytes, int Bf, int32_t* cfg_out, int cfg_cap, F body) {
+  CU(c, cudaSetDevice(c->device));
+  PackView pv;
+  std::vector<uint8_t> table;
+  TmpBufs T(c->stream);
+  if (pack) {
+    int r = parse_pack(c, pack, pack_bytes, 0, pv, table);
+    if (r) return r;
+    uint8_t* dev = (uint8_t*)T.get(pack_bytes);
+    if (!dev) return fail(c, 5410, "temporary allocation failed");
+    CU(c, cudaMemcpyAsync(dev, pack, pack_bytes, cudaMemcpyHostToDevice, c->stream));
+    pv.dev = dev;
+  }
+  Plan P;
+  P.Bf = P.Bx = Bf;
+  Arena meas;
+  meas.measure = true;
+  for (int pass = 0; pass < 2; ++pass) {
+    Arena* A = pass ? &P.arena : &meas;
+    if (pass && P.arena.init(meas.off + (1 << 20))) return fail(c, 5411, "cannot allocate %zu bytes of workspace", meas.off);
+    P.ops.clear();
+    Loader L{nullptr, c, &pv, A, c->stream};
+    PlanBuilder B{c, &P, A, Bf};
+    B.gn_partial = B.buf<float>(gn_scratch_floats(Bf, 32));
+    if (pass && B.gn_partial && gn_scratch_init(c->stream, B.gn_partial, Bf, 32)) return fail(c, 5007, "GroupNorm scratch init failed");
+    body(L, B);
+    if (L.err) return L.err;
+    if (B.err) return B.err;
+  }
+  int r = run_plan_ops(c, &P);
+  if (r) return r;
+  CU(c, cudaStreamSynchronize(c->stream));
+  // the configuration every igemm launch ran with (after igemm_launch's own adjustments)
+  int n = 0;
+  for (const Op& op : P.ops) {
+    if (op.kind != OP_IGEMM) continue;
+    if (cfg_out && n < cfg_cap) {
+      const IgemmParams& g = op.ig;
+      const int32_t v[SDXL_DBG_CFG_FIELDS] = {g.pair, g.CM, g.CN, g.a_split_dim, g.BN, g.nstages, g.epi_tma, g.epi_box_bytes};
+      memcpy(cfg_out + (size_t)n * SDXL_DBG_CFG_FIELDS, v, sizeof v);
+    }
+    ++n;
+  }
+  for (int i = n; cfg_out && i < cfg_cap; ++i)
+    for (int j = 0; j < SDXL_DBG_CFG_FIELDS; ++j) cfg_out[(size_t)i * SDXL_DBG_CFG_FIELDS + j] = -1;
+  return 0;
+}
+
+extern "C" int sdxl_dbg_plan_gemm(sdxl_ctx* c, int kind, const void* pack, size_t pack_bytes, int B, int H, int W, int Cin,
+                                  int Cout, int C2, const void* x, const void* x2, const float* bias_rows, int bias_ld,
+                                  int bias_off, const float* residual, void* out, int ldo, int32_t* cfg_out, int cfg_cap) {
+  if (!c || !pack || !x || !out || B < 1 || H < 1 || W < 1) return fail(c, -1, "sdxl_dbg_plan_gemm: bad argument");
+  switch (kind) {
+    case SDXL_DBG_CONV3:
+      return run_scratch_plan(c, pack, pack_bytes, B, cfg_out, cfg_cap, [&](Loader& L, PlanBuilder& P) {
+        const Conv cv = C2 ? L.conv("conv", Cin, Cout, 3, "skip", C2) : L.conv("conv", Cin, Cout, 3);
+        if (L.err) return;
+        ActView a{(const __half*)x, B, H, W, Cin}, sk{(const __half*)x2, B, H, W, C2};
+        P.conv3(a, C2 ? &sk : nullptr, cv, (float*)out, bias_rows ? bias_rows + bias_off : cv.b, bias_rows ? bias_ld : 0, residual);
+      });
+    case SDXL_DBG_UPCONV:
+      return run_scratch_plan(c, pack, pack_bytes, B, cfg_out, cfg_cap, [&](Loader& L, PlanBuilder& P) {
+        const Conv cv = L.upconv("conv", Cin, Cout);
+        __half* x16 = P.buf<__half>((size_t)B * H * W * Cin);
+        if (!L.err) P.upconv((const float*)x, B, H, W, cv, x16, (float*)out);
+      });
+    case SDXL_DBG_HEAD_HILO:
+      return run_scratch_plan(c, pack, pack_bytes, B, cfg_out, cfg_cap, [&](Loader& L, PlanBuilder& P) {
+        const Norm n = L.norm("norm", Cin);
+        const Conv cv = L.conv("conv", Cin, Cout, 3);
+        __half* w2 = L.dup_k(cv);
+        __half* y = P.buf<__half>((size_t)B * H * W * Cin);
+        __half* y_lo = P.buf<__half>((size_t)B * H * W * Cin);
+        if (!L.err) P.head_hilo((const float*)x, Cin, H, W, n, cv, w2, y, y_lo, (float*)out, ldo);
+      });
+    case SDXL_DBG_PADDED_S2:
+      if ((H & 1) || (W & 1)) return fail(c, 5412, "sdxl_dbg_plan_gemm: PaddedConv2d needs even H, W");
+      return run_scratch_plan(c, pack, pack_bytes, B, cfg_out, cfg_cap, [&](Loader& L, PlanBuilder& P) {
+        const Conv cv = L.conv("conv", Cin, Cout, 3);
+        __half* ph = P.buf<__half>((size_t)B * H * W * Cin);
+        if (!L.err) P.padded_conv_s2((const float*)x, B, H, W, cv, ph, (float*)out);
+      });
+    case SDXL_DBG_LINEAR:
+    case SDXL_DBG_LINEAR_F16:
+    case SDXL_DBG_GEGLU:
+      return run_scratch_plan(c, pack, pack_bytes, 1, cfg_out, cfg_cap, [&](Loader& L, PlanBuilder& P) {
+        const bool geglu = kind == SDXL_DBG_GEGLU;
+        const int gbn = geglu ? geglu_bn_for(Cout / 2) : 0;
+        if (geglu && (!gbn || (Cout & 1))) { L.err = fail(c, 5413, "sdxl_dbg_plan_gemm: GEGLU width %d not tileable", Cout); return; }
+        const Lin lin = L.linear("lin", Cin, Cout, true, gbn);
+        if (!L.err)
+          P.linear((const __half*)x, W, lin, geglu ? IGEMM_GEGLU : IGEMM_LINEAR, out, kind == SDXL_DBG_LINEAR, ldo,
+                   geglu ? nullptr : residual, ldo);
+      });
+  }
+  return fail(c, 5414, "sdxl_dbg_plan_gemm: unknown kind %d", kind);
+}
+
+extern "C" int sdxl_dbg_plan_group_norm(sdxl_ctx* c, const void* pack, size_t pack_bytes, const float* x1, int C1, const float* x2,
+                                        int C2, int B, int HW, int silu, sdxl_half* y, sdxl_half* raw, sdxl_half* y_lo) {
+  if (!c || !pack || !x1 || !y || B < 1 || HW < 1) return fail(c, -1, "sdxl_dbg_plan_group_norm: bad argument");
+  return run_scratch_plan(c, pack, pack_bytes, B, nullptr, 0, [&](Loader& L, PlanBuilder& P) {
+    const Norm n = L.norm("norm", C1 + (x2 ? C2 : 0));
+    if (!L.err) P.gn(x1, C1, x2, x2 ? C2 : 0, HW, n, silu, (__half*)y, (__half*)raw, (__half*)y_lo);
+  });
+}
+
+extern "C" int sdxl_dbg_plan_attention(sdxl_ctx* c, int small, const sdxl_half* q, int q_pitch, int q_col0, const sdxl_half* kv,
+                                       int kv_pitch, int k_col0, int v_col0, int B, int T, int S, int n_head, const sdxl_half* mask,
+                                       int causal, sdxl_half* out, int ldo) {
+  if (!c || !q || !kv || !out || B < 1 || T < 1 || S < 1 || n_head < 1) return fail(c, -1, "sdxl_dbg_plan_attention: bad argument");
+  return run_scratch_plan(c, nullptr, 0, B, nullptr, 0, [&](Loader&, PlanBuilder& P) {
+    if (small)
+      P.attn_small((const __half*)q, q_pitch, q_col0, (const __half*)kv, kv_pitch, k_col0, v_col0, T, S, n_head, (const __half*)mask,
+                   causal, (__half*)out, ldo);
+    else
+      P.attn((const __half*)q, q_pitch, q_col0, (const __half*)kv, kv_pitch, k_col0, v_col0, T, S, n_head, (__half*)out, ldo,
+             (float)(1.4426950408889634 / sqrt(64.0)));
+  });
+}
+
+extern "C" int sdxl_dbg_plan_vae_attention(sdxl_ctx* c, const sdxl_half* q, const sdxl_half* k, const sdxl_half* v, int T, int C,
+                                           float* scores, sdxl_half* probs, sdxl_half* vT, sdxl_half* out, int32_t* cfg_out,
+                                           int cfg_cap) {
+  if (!c || !q || !k || !v || !scores || !probs || !vT || !out) return fail(c, -1, "sdxl_dbg_plan_vae_attention: null argument");
+  if (T < 64 || T % 64 || C % 64) return fail(c, 5415, "sdxl_dbg_plan_vae_attention: T and C must be multiples of 64");
+  return run_scratch_plan(c, nullptr, 0, 1, cfg_out, cfg_cap, [&](Loader&, PlanBuilder& P) {
+    P.attn_single_head((const __half*)q, (const __half*)k, (const __half*)v, T, C, scores, (__half*)probs, (__half*)vT, (__half*)out);
+  });
 }

@@ -245,6 +245,18 @@ struct Loader {
     }
     return cv;
   }
+  // [O, 2*Ktot] = [W | W]: the weights of cv twice along K, for a conv over a hi/lo-split operand (PlanBuilder::head_hilo)
+  __half* dup_k(const Conv& cv) {
+    __half* w2 = A->get<__half>((size_t)cv.O * 2 * cv.Ktot);
+    if (!w2) { err = fail(c, 4005, "weight arena exhausted"); return nullptr; }
+    if (!A->measure)
+      for (int h2 = 0; h2 < 2; ++h2) {
+        cudaError_t e = cudaMemcpy2DAsync(w2 + (size_t)h2 * cv.Ktot, (size_t)2 * cv.Ktot * sizeof(__half), cv.w, (size_t)cv.Ktot * sizeof(__half),
+                                          (size_t)cv.Ktot * sizeof(__half), (size_t)cv.O, cudaMemcpyDeviceToDevice, st);
+        if (e != cudaSuccess) { err = fail(c, (int)e, "weight copy failed: %s", cudaGetErrorString(e)); return nullptr; }
+      }
+    return w2;
+  }
 };
 
 static int parse_pack(sdxl_ctx* c, const void* pack, size_t bytes, int on_device, PackView& pv,
@@ -441,11 +453,106 @@ struct PlanBuilder {
     igemm(a, skip, segs, cv.w, cv.O, cv.Ktot, a.H, a.W, a.Bn, IGEMM_LINEAR, 0, out, 1, cv.O, bias, bias_bstride, res, cv.O);
     add_flops(2.0 * a.Bn * a.H * a.W * (double)cv.O * (9.0 * cv.I + cv.I2));
   }
-  void gn(const float* x1, int C1, const float* x2, int C2, int HW, const Norm& n, int silu, __half* y, __half* raw) {
+  // PaddedConv2d (autoencoder/mod.rs:326-407): 3x3, stride 2, zero padding only past the bottom / right edge. Output (i, j) reads
+  // input rows 2i..2i+2 / cols 2j..2j+2 of x [Bn,H,W,I] f32 -> phase split into ph (f16, [4, Bn, H/2, W/2, I]), tap k: phase k&1,
+  // offset k>>1. out [Bn, H/2, W/2, O] f32.
+  void padded_conv_s2(const float* x, int Bn, int H, int W, const Conv& cv, __half* ph, float* out) {
+    if (err) return;
+    Op op{};
+    op.kind = OP_PHASE;
+    op.rs = {x, Bn, H, W, cv.I, ph};
+    P->ops.push_back(op);
+    const int H2 = H / 2, W2 = W / 2;
+    ActView a{ph, 4 * Bn, H2, W2, cv.I};
+    std::vector<IgemmSeg> segs;
+    for (int kh = 0; kh < 3; ++kh)
+      for (int kw = 0; kw < 3; ++kw)
+        segs.push_back({0, (int16_t)(kw >> 1), (int16_t)(kh >> 1), (int16_t)((((kh & 1) * 2) + (kw & 1)) * Bn), cv.Ipad / 64});
+    igemm(a, nullptr, segs, cv.w, cv.O, cv.Ktot, H2, W2, Bn, IGEMM_LINEAR, 0, out, 1, cv.O, cv.b, 0, nullptr, 0);
+    add_flops(2.0 * Bn * H2 * W2 * 9.0 * cv.I * cv.O);
+  }
+  // Output head GN -> SiLU -> 3x3 conv with the activation operand split hi + lo (y = f16(t), y_lo = f16(t - y)): the conv runs
+  // 18 tap segments over [y | y_lo] with the weights stored twice along K (w2 = Loader::dup_k(cv)), so it sees ~22 bits of t.
+  // x [Bf, HW, C] f32 -> out [Bf, HW, ldo] f32.
+  void head_hilo(const float* x, int C, int H, int W, const Norm& n, const Conv& cv, const __half* w2, __half* y, __half* y_lo,
+                 float* out, int ldo) {
+    gn(x, C, nullptr, 0, H * W, n, 1, y, nullptr, y_lo);
+    ActView a{y, Bf, H, W, C}, alo{y_lo, Bf, H, W, C};
+    std::vector<IgemmSeg> segs;
+    for (int part = 0; part < 2; ++part)   // K = [9 taps on hi | 9 taps on lo], weights [W | W]
+      for (int kh = 0; kh < 3; ++kh)
+        for (int kw = 0; kw < 3; ++kw) segs.push_back({(int16_t)part, (int16_t)(kw - 1), (int16_t)(kh - 1), 0, cv.Ipad / 64});
+    igemm(a, &alo, segs, w2, cv.O, 2 * cv.Ktot, H, W, Bf, IGEMM_LINEAR, 0, out, 1, ldo, cv.b, 0, nullptr, 0);
+    add_flops(2.0 * Bf * H * W * 9.0 * C * cv.O);
+  }
+  // Single-head attention of one image with d = Cm (autoencoder/mod.rs:572): S = q k^T (f32 [T,T]), P = softmax(S / sqrt(Cm))
+  // (f16), vT = v^T, out = P vT. q, k, v, out f16 [T, Cm]; T a multiple of 64.
+  void attn_single_head(const __half* q, const __half* k, const __half* v, int T, int Cm, float* S, __half* Pm, __half* vT,
+                        __half* out) {
+    if (err) return;
+    const int Kp = Loader::pad64(Cm);
+    {  // S = q k^T  (f32)
+      ActView a{q, 1, 1, T, Cm};
+      std::vector<IgemmSeg> segs{{0, 0, 0, 0, Kp / 64}};
+      igemm(a, nullptr, segs, k, T, Kp, 1, T, 1, IGEMM_LINEAR, 0, S, 1, T, nullptr, 0, nullptr, 0);
+      add_flops(2.0 * T * (double)T * Cm);
+    }
+    {
+      Op op{};
+      op.kind = OP_SOFTMAX;
+      op.sm = {S, (size_t)T, T, T, (float)(1.0 / sqrt((double)Cm)), Pm, (size_t)T};
+      P->ops.push_back(op);
+    }
+    {
+      Op op{};
+      op.kind = OP_TRANSPOSE;
+      op.tr = {v, (size_t)Cm, T, Cm, vT, (size_t)T};
+      P->ops.push_back(op);
+    }
+    {  // O = P v
+      ActView a{Pm, 1, 1, T, T};
+      std::vector<IgemmSeg> segs{{0, 0, 0, 0, T / 64}};
+      igemm(a, nullptr, segs, vT, Cm, T, 1, T, 1, IGEMM_LINEAR, 0, out, 0, Cm, nullptr, 0, nullptr, 0);
+      add_flops(2.0 * T * (double)T * Cm);
+    }
+  }
+  // Multi-head attention (head dim 64) on column windows of row-major f16 matrices: q at columns q_col0.. of [Bf*T, q_pitch],
+  // k / v at k_col0 / v_col0 of one [Bf*S, kv_pitch] matrix (fused QKV or KV GEMM outputs; one tensor map serves K and V).
+  void attn(const __half* qm, int q_pitch, int q_col0, const __half* kvm, int kv_pitch, int k_col0, int v_col0, int T,
+            int S, int n_head, __half* out, int ldo, float sl2e) {
+    if (err) return;
+    Op op{};
+    op.kind = OP_ATTN;
+    AttnParams& p = op.at;
+    p.T = T; p.S = S; p.n_head = n_head; p.B = Bf;
+    p.q_col0 = q_col0; p.k_col0 = k_col0; p.v_col0 = v_col0;
+    p.out = out; p.ldo = ldo; p.scale_log2e = sl2e;
+    if (!A->measure) {
+      int r = make_tmap_rows(&p.tmQ, qm, T, Bf, q_pitch, q_pitch);
+      if (!r) r = make_tmap_rows(&p.tmK, kvm, S, Bf, kv_pitch, kv_pitch);
+      if (!r) p.tmV = p.tmK;
+      if (r) { err = fail(c, r, "tensor map creation failed (attention)"); return; }
+    }
+    op.flops_exec = 4.0 * Bf * (double)((T + 127) / 128 * 128) * (double)((S + 127) / 128 * 128) * (n_head * 64);
+    P->ops.push_back(op);
+    add_flops(4.0 * Bf * T * (double)S * (n_head * 64));
+  }
+  // Masked / causal attention for short sequences (CUDA-core kernel), same column-window addressing as attn().
+  void attn_small(const __half* qm, int q_pitch, int q_col0, const __half* kvm, int kv_pitch, int k_col0, int v_col0, int T, int S,
+                  int n_head, const __half* mask, int causal, __half* out, int ldo) {
+    if (err) return;
+    Op op{};
+    op.kind = OP_ATTN_SMALL;
+    op.as = {qm, q_pitch, q_col0, kvm, kvm, kv_pitch, k_col0, v_col0, Bf, T, S, n_head, mask, causal, out, ldo};
+    P->ops.push_back(op);
+    add_flops(4.0 * Bf * T * (double)S * (n_head * 64));
+  }
+  void gn(const float* x1, int C1, const float* x2, int C2, int HW, const Norm& n, int silu, __half* y, __half* raw,
+          __half* y_lo = nullptr) {
     if (err) return;
     Op op{};
     op.kind = OP_GN;
-    op.gn = GnParams{x1, C1, x2, C2, Bf, HW, 32, n.g, n.b, n.eps, silu, y, raw, gn_partial, 0};
+    op.gn = GnParams{x1, C1, x2, C2, Bf, HW, 32, n.g, n.b, n.eps, silu, y, raw, gn_partial, 0, y_lo};
     P->ops.push_back(op);
   }
   void ln(const float* x, const Norm& n, int rows, __half* y) {

@@ -307,33 +307,9 @@ struct VaeStage {
     B.linear(s_gn1, M, aq, IGEMM_LINEAR, q16, 0, Cm, nullptr, 0);
     B.linear(s_gn1, M, ak, IGEMM_LINEAR, k16, 0, Cm, nullptr, 0);
     B.linear(s_gn1, M, av, IGEMM_LINEAR, v16, 0, Cm, nullptr, 0);
-    const int Kp = Loader::pad64(Cm);
     for (int b = 0; b < Bn && !B.err; ++b) {
       const size_t o = (size_t)b * T * Cm;
-      {  // S = q k^T  (f32)
-        ActView a{q16 + o, 1, 1, T, Cm};
-        std::vector<IgemmSeg> segs{{0, 0, 0, 0, Kp / 64}};
-        B.igemm(a, nullptr, segs, k16 + o, T, Kp, 1, T, 1, IGEMM_LINEAR, 0, S, 1, T, nullptr, 0, nullptr, 0);
-        B.add_flops(2.0 * T * (double)T * Cm);
-      }
-      {
-        Op op{};
-        op.kind = OP_SOFTMAX;
-        op.sm = {S, (size_t)T, T, T, (float)(1.0 / sqrt((double)Cm)), Pm, (size_t)T};
-        P->ops.push_back(op);
-      }
-      {
-        Op op{};
-        op.kind = OP_TRANSPOSE;
-        op.tr = {v16 + o, (size_t)Cm, T, Cm, vT, (size_t)T};
-        P->ops.push_back(op);
-      }
-      {  // O = P v
-        ActView a{Pm, 1, 1, T, T};
-        std::vector<IgemmSeg> segs{{0, 0, 0, 0, T / 64}};
-        B.igemm(a, nullptr, segs, vT, Cm, T, 1, T, 1, IGEMM_LINEAR, 0, ao + o, 0, Cm, nullptr, 0, nullptr, 0);
-        B.add_flops(2.0 * T * (double)T * Cm);
-      }
+      B.attn_single_head(q16 + o, k16 + o, v16 + o, T, Cm, S, Pm, vT, ao + o);
     }
     B.linear(ao, M, aproj, IGEMM_LINEAR, other(), 1, Cm, x(), Cm);  // x + proj_out(attn)
     flip();
@@ -473,23 +449,10 @@ static int build_vae_enc_plan(sdxl_vae* v, Plan* P, Arena* A) {
     st.vres(b.r[0]);
     st.vres(b.r[1]);
     if (b.down) {
-      // PaddedConv2d(3x3, stride 2, padding (left 0, right 1, top 0, bottom 1)), autoencoder/mod.rs:326-407: output (i, j) reads
-      // input rows 2i..2i+2 / cols 2j..2j+2 with zeros past the bottom/right edge -> tap k: phase k&1, offset k>>1.
-      Op op{};
-      op.kind = OP_PHASE;
-      op.rs = {st.x(), Bn, st.H, st.W, b.Cout, s_ph};
-      P->ops.push_back(op);
-      const int H2 = st.H / 2, W2 = st.W / 2;
-      ActView a{s_ph, 4 * Bn, H2, W2, b.Cout};
-      std::vector<IgemmSeg> segs;
-      for (int kh = 0; kh < 3; ++kh)
-        for (int kw = 0; kw < 3; ++kw)
-          segs.push_back({0, (int16_t)(kw >> 1), (int16_t)(kh >> 1), (int16_t)((((kh & 1) * 2) + (kw & 1)) * Bn), b.downc.Ipad / 64});
-      B.igemm(a, nullptr, segs, b.downc.w, b.downc.O, b.downc.Ktot, H2, W2, Bn, IGEMM_LINEAR, 0, st.other(), 1, b.downc.O, b.downc.b, 0,
-              nullptr, 0);
-      B.add_flops(2.0 * Bn * H2 * W2 * 9.0 * b.Cout * b.downc.O);
+      // PaddedConv2d(3x3, stride 2, padding (left 0, right 1, top 0, bottom 1)), autoencoder/mod.rs:326-407
+      B.padded_conv_s2(st.x(), Bn, st.H, st.W, b.downc, s_ph, st.other());
       st.flip();
-      st.H = H2; st.W = W2;
+      st.H /= 2; st.W /= 2;
     }
   }
   if (B.err) return B.err;

@@ -86,6 +86,10 @@ PROTOTYPES = {
     "sdxl_dbg_igemm_timeline": (I, [P, I, I, I, I, I, C.POINTER(C.c_uint64)]),
     "sdxl_dbg_igemm_gaps": (I, [P, I, I, I, I, I, C.POINTER(C.c_int64)]),
     "sdxl_dbg_attention_timeline": (I, [P, I, I, I, I, C.POINTER(C.c_longlong)]),
+    "sdxl_dbg_plan_gemm": (I, [P, I, P, C.c_size_t, I, I, I, I, I, I, P, P, P, I, I, P, P, I, C.POINTER(C.c_int32), I]),
+    "sdxl_dbg_plan_group_norm": (I, [P, P, C.c_size_t, P, I, P, I, I, I, I, P, P, P]),
+    "sdxl_dbg_plan_attention": (I, [P, I, P, I, I, P, I, I, I, I, I, I, I, P, I, P, I]),
+    "sdxl_dbg_plan_vae_attention": (I, [P, P, P, P, I, I, P, P, P, P, C.POINTER(C.c_int32), I]),
     "sdxl_randn": (I, [P, P, C.c_size_t, C.c_uint64, C.c_uint64]),
     "sdxl_qkv_attention": (I, [P, P, P, P, P, I, I, I, I, I, P]),
     "sdxl_op_linear": (I, [P, P, P, P, P, I, I, I, I, I, P]),
